@@ -1,6 +1,6 @@
 """bench.py — vectors quantized / second at dim=256, codebook=1024 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload cfg2|cfg5]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload cfg2|cfg5] [--dump-outputs DIR]
 
 Workload (N=1 and per GPU for N>1): BASELINE.json configs[1] — VectorQuantize(dim=256, codebook_size=1024),
 x = (64, 4096, 256) bf16, training-mode forward with the EMA codebook update.  A "step" is one such
@@ -14,6 +14,11 @@ barrier kernel; ONE NCCL all-reduce if symmetric memory is unavailable); the tim
 VectorQuantize(dim=256, codebook_size=1024) training-mode forward on the full 262144-vector batch — and falls back
 to the torch-CPU oracle port (oracle/vq_oracle_torch.py, the same ATen op sequence) only if the package cannot be
 imported, saying so in `cpu_baseline.kind`.
+
+`--dump-outputs DIR` writes what the last headline-timed step returned (rank 0's shard under torchrun) as float32 .npy
+files: `indices` and `loss` whole, and `quantize_rows`, a fixed seeded sample of the quantized rows (their row numbers in
+`quantize_row_ids`, float64).  Inputs and codebooks are seeded, so two builds run with the same arguments can be compared
+output for output.
 """
 import argparse
 import json
@@ -31,6 +36,21 @@ METRIC = "vectors quantized/sec at dim=256, codebook=1024; indices bit-exact vs 
 B, T, D, K = 64, 4096, 256, 1024
 WORKLOAD = "VectorQuantize dim=256 codebook_size=1024, x=(64,4096,256) bf16, EMA on (BASELINE.json configs[1])"
 E2E_CHUNKS = int(os.environ.get("VQB_E2E_CHUNKS", "10"))  # row chunks of the host-buffer pipeline (forward_host)
+DUMP_ROWS = 16384   # quantized rows sampled by --dump-outputs: 16 MB at D=256 in float32 (all of q would be 256 MB)
+
+
+def dump_outputs(out_dir, q, ind, loss):
+    """Write one step's outputs to out_dir as .npy: indices and loss whole, a fixed seeded sample of the quantized rows."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    rows = q.detach().reshape(-1, q.shape[-1])
+    pick = torch.randperm(rows.shape[0], generator=torch.Generator().manual_seed(0))[:DUMP_ROWS].sort().values
+    arrays = {"quantize_rows": rows[pick.to(rows.device)].float(), "quantize_row_ids": pick.double(),
+              "indices": ind.float(),   # exact: codebook indices are far below 2**24
+              "loss": loss.detach().float()}
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.cpu().numpy())
 
 
 def load_peaks():
@@ -126,7 +146,7 @@ def run_reference_arm(args):
     # torchrun exports OMP_NUM_THREADS=1 for its workers; the reference arm is entitled to every host thread
     for var in ("OMP_NUM_THREADS", "MKL_NUM_THREADS"):
         os.environ.pop(var, None)
-    steps = max(1, min(args.steps, 5))
+    steps = args.steps
     warm = max(1, min(args.warmup, 2))
     v, ms = time_cpu(steps, warm)
     line = {
@@ -341,6 +361,8 @@ def run_gpu_arm(args):
     clocks = sampler.stop(t_start, t_end)
     ms_dev = max_over_ranks(e0.elapsed_time(e1) / args.steps)
     host_ms = (t_host - t_start) * 1e3 / args.steps   # CPU time to enqueue one step (must stay below ms_dev)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, q, ind, loss)
 
     # ---------------- the dominant kernel's launch duration (roofline): the same K steps once more, now with a CUDA
     # event pair recorded on the launching stream around vq_assign_kernel.  Kept out of the headline region because
@@ -484,7 +506,12 @@ def main():
                     help="cfg2 = BASELINE.json configs[1] (the headline, default); cfg5 = configs[4], GroupedResidualVQ, strong scaling")
     ap.add_argument("--no-sustained", action="store_true", help="skip the >= 2 s sustained-clock block")
     ap.add_argument("--sustained-seconds", type=float, default=2.0)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs to DIR as .npy files")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the GPU path (--impl ours)")
     args.warmup = max(args.warmup, 3)
     if args.impl == "reference":
         run_reference_arm(args)

@@ -351,7 +351,37 @@ def dropout_cases():
         print(f"{name}: {os.path.getsize(path) / 1024:.0f} KiB", [int((store[f's{i}_indices'][0, 0] >= 0).sum()) for i in range(len(steps))])
 
 
+STATE_DICT_CASES = [
+    ("VectorQuantize", dict(dim=64, codebook_size=32, use_cosine_sim=True)),
+    ("ResidualVQ", dict(dim=32, num_quantizers=3, codebook_size=16)),
+    ("VectorQuantize", dict(dim=64, codebook_size=32, heads=4, codebook_dim=16)),
+    ("VectorQuantize", dict(dim=48, codebook_size=32, heads=2, separate_codebook_per_head=True)),
+    ("SimVQ", dict(dim=32, codebook_size=40)),
+    ("GroupedResidualVQ", dict(dim=64, groups=2, num_quantizers=2, codebook_size=16, shared_codebook=True)),
+]
+
+
+def state_dict_cases():
+    """The reference's freshly constructed state_dict (torch.manual_seed(0) before construction) for each entry of
+    STATE_DICT_CASES: key order in meta, every tensor as stored, so that checkpoint loading is checked without the reference."""
+    ref = load_reference()
+    store, meta = {}, []
+    for i, (cls, kw) in enumerate(STATE_DICT_CASES):
+        torch.manual_seed(0)
+        sd = getattr(ref, cls)(**kw).state_dict()
+        for k, v in sd.items():
+            store[f"c{i}/{k}"] = v.detach().cpu().numpy()
+        meta.append(dict(cls=cls, kw=kw, keys=list(sd)))
+    store["meta"] = np.frombuffer(json.dumps(dict(cases=meta, torch=torch.__version__)).encode(), dtype=np.uint8)
+    path = os.path.join(OUT, "state_dict", "reference_init.npz")
+    os.makedirs(os.path.dirname(path), exist_ok=True)
+    np.savez_compressed(path, **store)
+    print(f"{path}: {os.path.getsize(path) / 1024:.0f} KiB")
+
+
 def main():
+    if "--state-dict" in sys.argv:
+        return state_dict_cases()
     if "--dropout" in sys.argv:
         return dropout_cases()
     if "--mask-rvq" in sys.argv:

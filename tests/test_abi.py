@@ -89,27 +89,23 @@ def test_state_dict_layout_matches_reference():
     assert "rvqs.1.layers.1._codebook.cluster_size" in g.state_dict()
 
 
-def test_reference_state_dict_loads(tmp_path):
-    """If the reference is importable here, its state_dict must load into ours key-for-key."""
-    from oracle.ref_loader import reference_available, load_reference
-    if not reference_available():
-        pytest.skip("reference tree not present on this machine")
-    ref = load_reference()
+def test_reference_state_dict_loads():
+    """The reference's state_dict must load into ours key-for-key.  tests/golden/state_dict/reference_init.npz holds the
+    reference's freshly constructed state_dicts under torch.manual_seed(0) (oracle/gen_golden.py --state-dict)."""
+    import json
+    import numpy as np
     import vector_quantize_pytorch_b200 as m
-    for build in (lambda mod: mod.VectorQuantize(dim=64, codebook_size=32, use_cosine_sim=True),
-                  lambda mod: mod.ResidualVQ(dim=32, num_quantizers=3, codebook_size=16),
-                  lambda mod: mod.VectorQuantize(dim=64, codebook_size=32, heads=4, codebook_dim=16),
-                  lambda mod: mod.VectorQuantize(dim=48, codebook_size=32, heads=2, separate_codebook_per_head=True),
-                  lambda mod: mod.SimVQ(dim=32, codebook_size=40),
-                  lambda mod: mod.GroupedResidualVQ(dim=64, groups=2, num_quantizers=2, codebook_size=16, shared_codebook=True)):
+    z = np.load(os.path.join(ROOT, "tests", "golden", "state_dict", "reference_init.npz"))
+    cases = json.loads(bytes(z["meta"]).decode())["cases"]
+    assert len(cases) == 6
+    for i, case in enumerate(cases):
+        sa = {k: torch.from_numpy(z[f"c{i}/{k}"]) for k in case["keys"]}
         torch.manual_seed(0)
-        a = build(ref)
-        torch.manual_seed(0)
-        b = build(m)
-        sa, sb = a.state_dict(), b.state_dict()
-        assert list(sa) == list(sb)
+        b = getattr(m, case["cls"])(**case["kw"])
+        sb = b.state_dict()
+        assert list(sa) == list(sb), case
         for k in sa:  # same RNG consumption at construction -> identical initial codebooks
-            assert torch.equal(sa[k], sb[k]), k
+            assert torch.equal(sa[k], sb[k]), (case, k)
         b.load_state_dict(sa)
 
 
